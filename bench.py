@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps K --warmup W            # this engine, 1 GPU
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...   # N GPUs, weak scaling
     python bench.py --impl reference ...                      # the reference algorithm on the host CPUs
+    python bench.py ... --dump-outputs DIR                    # + the last timed step's arrays as DIR/*.npy (A/B of builds)
 
 One "step" = one lockstep vector step (action -> state', obs, reward, terminated, truncated, autoreset) of the
 whole batch. Headline workload (config.workload): BASELINE.json configs[2], MiniGrid-DoorKey-8x8-v0 with 262144
@@ -31,6 +32,7 @@ ALGO_BYTES_PER_STEP = 348  # SURVEY.md 8(d): action 4 + patch 147 + obs 147 + re
 L2_BYTES = 126e6
 HEADLINE_ENV = "MiniGrid-DoorKey-8x8-v0"
 # BASELINE.json configs[1], [3], [4] (per-GPU share); configs[0] (Empty-5x5, 1 env, CPU) is the `config1` key
+DUMP_ENVS = 65536  # --dump-outputs: at most this many environments of the last step
 OTHER_CONFIGS = [("MiniGrid-Empty-8x8-v0", 65536), ("MiniGrid-LavaCrossingS9N1-v0", 262144), ("MiniGrid-FourRooms-v0", 262144)]
 
 
@@ -50,7 +52,26 @@ def parse_args():
     ap.add_argument("--graph", type=int, default=1, help="replay the step loop as CUDA graphs (0 = eager launches)")
     ap.add_argument("--sync-episodes", action="store_true", help="do NOT desynchronise the episodes (round-1 behaviour: no autoreset in the timed region)")
     ap.add_argument("--host-format", default="packed", choices=["packed", "full"], help="D2H format of the e2e leg (packed: 52 B/env expanded on the host)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned as DIR/<name>.npy "
+                    "(float32, reward float64; a fixed sample of DUMP_ENVS environments of larger batches) to compare two builds")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, env, seed=0):
+    """Writes the arrays env.step() returned last: step() hands back the same tensors on every call (the copy=False
+    convention), so after the timed loop they hold its last step. Batches above DUMP_ENVS envs are sampled, the same
+    sorted subset of env indices on every run (65536 envs: 39 MB of float32 images)."""
+    import torch
+
+    n = env.num_envs
+    idx = np.arange(n) if n <= DUMP_ENVS else np.sort(np.random.default_rng(seed).choice(n, DUMP_ENVS, replace=False))
+    sel = torch.as_tensor(idx, device=env.device)
+    outputs = {"image": (env._obs_dict["image"], torch.float32), "direction": (env._obs_dict["direction"], torch.float32),
+               "reward": (env._reward, torch.float64), "terminated": (env._terminated, torch.float32),
+               "truncated": (env._truncated, torch.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, dtype) in outputs.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.index_select(0, sel).to(dtype).cpu().numpy())
 
 
 def load_peaks():
@@ -372,6 +393,9 @@ def main():
             launches += (K // G) * G  # launches replayed by the graphs (each captured step() is one kernel node)
             if graph_rem is not None:
                 launches += K % G
+        # the batch that took the last timed step: graphs replay the steps t = 0 .. K-1 they were captured with (the
+        # remainder graph its tail), eager launches continue from t = W
+        last_batch = ((K if graph is not None else W + K) - 1) % R
         for b in batches:
             b.check_actions()
         # share of envs that were regenerated per timed step (pending flags after the run, averaged over the batches)
@@ -379,7 +403,7 @@ def main():
         res = {"env": env_id, "envs_per_gpu": n, "total_envs": total, "steps": K, "ms": ms, "ms_per_step": ms / K,
                "value": total * K / (ms * 1e-3), "launches": int(launches), "R": R, "ws": ws, "G": G, "graph": graph is not None,
                "graph_error": graph_error, "clocks": clocks, "host_enqueue_us_per_step": 1e6 * host_enqueue_s / K,
-               "autoreset_fraction_per_step": pend}
+               "autoreset_fraction_per_step": pend, "last_batch": last_batch}
         achieved = ALGO_BYTES_PER_STEP * n / (ms / K * 1e-3) / 1e9
         res["achieved_gbs"], res["frac"] = achieved, achieved / peak
         return res, batches, (eager_run, act_rows, step_fns, T, R)
@@ -391,6 +415,8 @@ def main():
                                                                          sync_episodes=args.sync_episodes, want_graph=bool(args.graph))
     ms, launches = head["ms"], head["launches"]
     value = head["value"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batches[head["last_batch"]])
 
     # per-launch events (perturbs the stream; reported, not used for the headline)
     kstep_ms = ms / K if launches == K else None

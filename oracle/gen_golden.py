@@ -4,6 +4,9 @@ Run:  python -m oracle.gen_golden          (needs /root/reference; see oracle/re
 
 Run:  python -m oracle.gen_golden next     (only the next_rollout_* fixtures of generators that have no device kernel yet)
 
+Run:  python -m oracle.gen_golden traces   (only traces_reference.npz: the reference's side of the scenarios of
+                                           tests/test_oracle_vs_reference.py and tests/test_oracle_next.py)
+
 Two families of fixtures, both produced by the reference's own MiniGridEnv objects:
   rollout_<id>.npz   seeded reset + T lockstep steps of N envs with SyncVectorEnv NEXT_STEP
                      autoreset, uniform-random actions (np.random.default_rng(1234)); records every
@@ -263,6 +266,67 @@ def main_next():
         print("next_rollout", env_id, "episodes ended:", int((d["terminated"] | d["truncated"]).sum()))
 
 
+def main_traces():
+    """Every scenario of tests/test_oracle_vs_reference.py and tests/test_oracle_next.py run on the reference's env
+    objects with a recording trace (oracle/trace.py), under the names the tests replay."""
+    sys.path.insert(0, os.path.join(os.path.dirname(HERE), "tests"))
+    import test_oracle_next as tn
+    import test_oracle_vs_reference as tv
+
+    from oracle import trace
+    from oracle.oracle import ENV_SPECS, NEXT_SPECS
+
+    gym, _ = load()
+    from minigrid.wrappers import DictObservationSpaceWrapper
+
+    def make(env_id, n, autoreset="next_step", spec=None, gym_kwargs=None, no_death=(), death_cost=-1.0, bonus=None):
+        wrap = reward_wrap(no_death, death_cost, bonus) if (no_death or bonus) else None
+        return ReferenceVecEnv(env_id, n, autoreset=autoreset, wrap=wrap, **(gym_kwargs or {}))
+
+    out = {}
+
+    def record(name, scenario, *args):
+        t = trace.Trace(name)
+        scenario(make, t, *args)
+        out[name] = t.close()
+
+    def registry(make, t):
+        for env_id in ENV_SPECS:
+            e = gym.make(env_id).unwrapped
+            t.exact(env_id, [e.width, e.height, e.max_steps, e.see_through_walls])
+
+    def dict_observation(make, t):
+        words = DictObservationSpaceWrapper.get_minigrid_words()
+        assert sorted(words.values()) == list(range(len(words)))
+        t.exact("words", sorted(words, key=words.get))
+        for env_id in tv.constant_mission_ids():
+            obs, _ = DictObservationSpaceWrapper(gym.make(env_id)).reset(seed=0)
+            t.exact(f"mission {env_id}", obs["mission"])
+
+    for mode in ("next_step", "same_step"):
+        for env_id in ENV_SPECS:
+            record(f"lockstep {env_id} {mode}", tv.lockstep, env_id, mode)
+        for env_id in NEXT_SPECS:
+            record(f"next lockstep {env_id} {mode}", tv.lockstep, env_id, mode, 5, 420, 2024, 78)
+        for env_id, no_death, bonus in tv.REWARD_WRAPPER_CASES:
+            record(f"reward wrappers {env_id} {mode}", tv.reward_wrappers, env_id, no_death, bonus, mode)
+    record("registry", registry)
+    record("dict observation", dict_observation)
+    for case in tv.UNREGISTERED_SIZES:
+        record(f"unregistered {case[0]} {case[2]}", tv.unregistered_size, *case)
+    for env_id in tv.WRAPPER_IDS:
+        record(f"observation wrappers {env_id}", tv.observation_wrappers, env_id)
+    for env_id in tn.MEMORY_IDS:
+        record(f"memory cells {env_id}", tn.memory_cells, env_id)
+    for env_id in tn.ROOMGRID_IDS:
+        record(f"roomgrid post-filters {env_id}", tn.roomgrid_post_filters, env_id)
+    for env_id in tn.BOX_IDS:
+        record(f"boxes {env_id}", tn.boxes_hide_keys, env_id)
+    os.makedirs(OUT, exist_ok=True)
+    trace.save(os.path.join(OUT, "traces_reference.npz"), out)
+    print("traces", len(out), "scenarios")
+
+
 def main():
     os.makedirs(OUT, exist_ok=True)
     for env_id, (n, t, seed) in ROLLOUTS.items():
@@ -292,8 +356,11 @@ if __name__ == "__main__":
         main_wrappers()
     elif sys.argv[1:] == ["reward_wrappers"]:
         main_reward_wrappers()
+    elif sys.argv[1:] == ["traces"]:
+        main_traces()
     else:
         main()
         main_next()
         main_wrappers()
         main_reward_wrappers()
+        main_traces()

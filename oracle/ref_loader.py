@@ -1,9 +1,8 @@
-"""Import the UNMODIFIED Python reference (TEST INFRASTRUCTURE ONLY, build container only).
+"""Import the UNMODIFIED Python reference (TEST INFRASTRUCTURE ONLY).
 
-/root/reference is read-only and exists only in the build container (never on the GPU box), so
-everything that uses this module is skipped when the tree is absent. gymnasium and pygame are not
-installed in the image: oracle/ref_shim supplies import stand-ins (our own code); a real gymnasium,
-if ever installed, takes precedence.
+Only the fixture generators (oracle/gen_golden.py) use this module; the tests read what they recorded under
+tests/golden/ and never need the reference. gymnasium and pygame may be missing: oracle/ref_shim supplies import
+stand-ins (our own code); a real gymnasium, if installed, takes precedence.
 """
 from __future__ import annotations
 
@@ -49,6 +48,8 @@ class ReferenceVecEnv:
         self.envs = [gym.make(env_id, **kwargs).unwrapped for _ in range(num_envs)]
         self.wrapped = [wrap(e) for e in self.envs] if wrap is not None else self.envs
         self.num_envs = num_envs
+        e0 = self.envs[0]
+        self.width, self.height, self.max_steps, self.see_through = e0.width, e0.height, e0.max_steps, e0.see_through_walls
         self.autoreset = autoreset
         self.pending = [False] * num_envs
 
@@ -98,6 +99,15 @@ class ReferenceVecEnv:
             m = (1 << 64) - 1
             rng[i] = [s >> 64, s & m, inc >> 64, inc & m, st["has_uint32"], st["uinteger"]]
         return {"grid": grid, "agent": agent, "rng": rng, "pending": np.asarray(self.pending, np.uint8)}
+
+    def set_state(self, agent):
+        """Agent records as OracleVecEnv.set_state takes them: x, y, dir, carried object type / colour (-1: none),
+        step_count."""
+        from minigrid.core.world_object import WorldObj
+
+        for e, (x, y, d, ctype, ccolor, steps) in zip(self.envs, self.np.asarray(agent).tolist()):
+            e.agent_pos, e.agent_dir, e.step_count = (x, y), d, steps
+            e.carrying = None if ctype < 0 else WorldObj.decode(ctype, ccolor, 0)
 
     def full_obs(self):
         from minigrid.wrappers import FullyObsWrapper

@@ -1,15 +1,16 @@
 """SURVEY 8(f) rows restated in the oracle ahead of their device kernels (f-1: LockedRoom, Playground; f-2, the first
 step post-filter: GoToDoor): the oracle
-against fixtures produced by the Python reference (travels to any box) and, where /root/reference exists, against
-the live reference. The product does not register these ids yet, so there is no GPU counterpart of this file."""
+against fixtures produced by the Python reference and against recordings of the reference's side of the scenarios
+below (tests/golden/traces_reference.npz). The product does not register these ids yet, so there is no GPU counterpart
+of this file."""
 import os
 
 import numpy as np
 import pytest
 from conftest import golden_files
 from test_oracle_golden import test_rollout_matches_reference_fixture as check_rollout_fixture
+from test_oracle_vs_reference import lockstep, replay
 
-from oracle import ref_loader
 from oracle.oracle import ENV_SPECS, NEXT_SPECS, OracleVecEnv
 
 
@@ -27,28 +28,10 @@ def test_next_ids_are_not_product_ids_yet():
             specs.get(env_id)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
 @pytest.mark.parametrize("env_id", list(NEXT_SPECS))
 @pytest.mark.parametrize("mode", ["next_step", "same_step"])
 def test_next_lockstep_rollout_against_live_reference(env_id, mode):
-    n, t_steps = 5, 420
-    ref = ref_loader.ReferenceVecEnv(env_id, n, autoreset=mode)
-    orc = OracleVecEnv(env_id, n, autoreset=mode)
-    e0 = ref.envs[0]
-    assert (orc.width, orc.height, orc.max_steps, orc.see_through) == (e0.width, e0.height, e0.max_steps, e0.see_through_walls)
-    ro, rd = ref.reset(seed=2024)
-    oo, od = orc.reset(seed=2024)
-    np.testing.assert_array_equal(ro, oo)
-    np.testing.assert_array_equal(rd, od)
-    rng = np.random.default_rng(78)
-    for t in range(t_steps):
-        a = rng.integers(0, 7, n)
-        for x, y, name in zip(ref.step(a), orc.step(a), ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=f"{name} t={t}")
-    rs, os_ = ref.get_state(), orc.get_state()
-    for k in rs:
-        np.testing.assert_array_equal(rs[k], os_[k], err_msg=k)
-    np.testing.assert_array_equal(ref.full_obs(), orc.full_obs())
+    replay(f"next lockstep {env_id} {mode}", lockstep, env_id, mode, 5, 420, 2024, 78)
 
 
 # ---- the device generators of these kinds (mg_levels.cuh), compiled for the CPU by tests/host_emu ----
@@ -86,44 +69,31 @@ def test_next_device_generators_lockstep_vs_oracle(env_id, mode, n):
     parity.check_lockstep_vs_oracle(emu, orc, 450, seed=99, check_state_every=150)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-@pytest.mark.parametrize("env_id", ["MiniGrid-MemoryS7-v0", "MiniGrid-MemoryS13Random-v0"])
-def test_memory_success_and_failure_cells_against_live_reference(env_id):
+# ---- the post-filter branches random actions never reach, driven on purpose (scenarios as in test_oracle_vs_reference) ----
+def memory_cells(make, trace, env_id):
     """Random actions almost never walk the hallway: drive every env to its end, half of them up and half down, so that
-    both post-filter branches (memory.py:156-164) fire in the reference and in the oracle."""
+    both post-filter branches (memory.py:156-164) fire."""
     n = 24
-    ref = ref_loader.ReferenceVecEnv(env_id, n)
-    orc = OracleVecEnv(env_id, n)
-    np.testing.assert_array_equal(ref.reset(seed=300)[0], orc.reset(seed=300)[0])
-    size = ref.envs[0].width
+    env = make(env_id, n)
+    trace.reset(env.reset(seed=300))
+    size = env.width
     turn = np.where(np.arange(n) % 2 == 0, 0, 1)  # left = up, right = down
     script = [np.full(n, 2)] * size + [turn] + [np.full(n, 2)] * 2 + [np.full(n, 3)] * 2
     rewards, ended = [], 0
     for a in script * 2:  # the second pass runs on the autoreset episodes
-        r, q = ref.step(a), orc.step(a)
-        for x, y, name in zip(r, q, ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=name)
-        rewards.append(np.asarray(r[2]))
+        r = trace.step(env.step(a), a)
+        rewards.append(np.array(r[2]))  # a copy: the oracle reuses its output buffers
         ended += int(np.asarray(r[3]).sum())
     rewards = np.concatenate(rewards)
     assert ended >= n and (rewards > 0).any() and ended > int((rewards > 0).sum())  # successes and failures both seen
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-@pytest.mark.parametrize("env_id", ["MiniGrid-Unlock-v0", "MiniGrid-UnlockPickup-v0", "MiniGrid-BlockedUnlockPickup-v0",
-                                    "MiniGrid-KeyCorridorS3R3-v0", "MiniGrid-KeyCorridorS6R3-v0"])
-def test_roomgrid_post_filters_fire_against_live_reference(env_id):
-    """Random actions practically never unlock a door or reach the object behind it: put every agent next to its target
-    (the same injection in the reference's env objects and in the oracle) so that the success branches of unlock.py:88-96
-    and of the `carrying == self.obj` filters run in both."""
-    n = 16
-    ref = ref_loader.ReferenceVecEnv(env_id, n)
-    orc = OracleVecEnv(env_id, n)
-    np.testing.assert_array_equal(ref.reset(seed=700)[0], orc.reset(seed=700)[0])
-    from minigrid.core.world_object import Key
+def _roomgrid_targets(ref, unlock):
+    """From the reference's env objects: every agent next to its target (Unlock: in front of the locked door, with its
+    key; the pickup variants: facing the object). Returns the agent records and how many envs were moved."""
+    from minigrid.core.constants import COLOR_TO_IDX
 
-    agent = orc.get_state()["agent"].copy()
-    unlock = env_id == "MiniGrid-Unlock-v0"
+    agent = ref.get_state()["agent"].copy()
     moved = 0
     for i, e in enumerate(ref.envs):
         tx, ty = (e.door.cur_pos if unlock else e.obj.cur_pos)
@@ -131,48 +101,68 @@ def test_roomgrid_post_filters_fire_against_live_reference(env_id):
             ax, ay = tx - dx, ty - dy
             here = e.grid.get(ax, ay) if 0 < ax < e.width - 1 and 0 < ay < e.height - 1 else False
             if here is None or (here and here.type == "door" and not unlock):  # (S3 rooms: the only free neighbour is the doorway)
-                e.agent_pos, e.agent_dir = (ax, ay), d
-                e.carrying = Key(e.door.color) if unlock else None
                 agent[i, :3] = (ax, ay, d)
-                agent[i, 3:5] = (5, {"red": 0, "green": 1, "blue": 2, "purple": 3, "yellow": 4, "grey": 5}[e.door.color]) if unlock else (-1, 0)
+                agent[i, 3:5] = (5, COLOR_TO_IDX[e.door.color]) if unlock else (-1, 0)
                 moved += 1
                 break
+    return agent, moved
+
+
+def roomgrid_post_filters(make, trace, env_id):
+    """Random actions practically never unlock a door or reach the object behind it: put every agent next to its target
+    (the same injection on both sides) so that the success branches of unlock.py:88-96 and of the `carrying == self.obj`
+    filters run."""
+    n = 16
+    env = make(env_id, n)
+    trace.reset(env.reset(seed=700))
+    unlock = env_id == "MiniGrid-Unlock-v0"
+    targets = _roomgrid_targets(env, unlock) if trace.recording else None
+    agent = trace.input("injected agent", lambda: targets[0])
+    moved = int(trace.input("moved", lambda: targets[1]))
     assert moved >= n // 2
-    orc.set_state(agent=agent)
+    env.set_state(agent=agent)
     act = np.full(n, 5 if unlock else 3)
     ended = 0
     for a in (act, act, np.full(n, 2)):
-        r, q = ref.step(a), orc.step(a)
-        for x, y, name in zip(r, q, ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=name)
+        r = trace.step(env.step(a), a)
         ended += int((np.asarray(r[3]) & (np.asarray(r[2]) > 0)).sum())
     assert ended >= moved  # every injected env succeeded once
-    rs, os_ = ref.get_state(), orc.get_state()
-    for k in rs:
-        np.testing.assert_array_equal(rs[k], os_[k], err_msg=k)
+    trace.state(env, full_obs=False)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
-@pytest.mark.parametrize("env_id", ["MiniGrid-ObstructedMaze-1Dlh-v0", "MiniGrid-ObstructedMaze-Full-v1"])
-def test_boxes_hide_keys_against_live_reference(env_id):
-    """Box.contains / Box.toggle (world_object.py:273-293) in the oracle: agents put in front of a box in the reference's
-    env objects and in the oracle, then toggle / pick up / drop scripts."""
+def boxes_hide_keys(make, trace, env_id):
+    """Box.contains / Box.toggle (world_object.py:273-293): agents put in front of a box, then toggle / pick up / drop
+    scripts."""
     n = 24
-    ref = ref_loader.ReferenceVecEnv(env_id, n)
-    orc = OracleVecEnv(env_id, n)
-    np.testing.assert_array_equal(ref.reset(seed=11)[0], orc.reset(seed=11)[0])
-    agent, moved = parity.face_first_cell_of_type(orc, 7)
+    env = make(env_id, n)
+    trace.reset(env.reset(seed=11))
+    agent, moved = parity.face_first_cell_of_type(env, 7)
     assert moved.sum() >= n // 2
-    for i, e in enumerate(ref.envs):
-        e.agent_pos, e.agent_dir, e.carrying = (int(agent[i, 0]), int(agent[i, 1])), int(agent[i, 2]), None
-    orc.set_state(agent=agent)
+    env.set_state(agent=trace.exact("injected agent", agent))
     half = np.arange(n) % 2 == 0
     script = [np.where(half, 5, 3), np.where(half, 3, 0), np.where(half, 6, 4), np.where(half, 6, 5), np.where(half, 4, 3), np.full(n, 2)]
     for a in script:
-        r, q = ref.step(a), orc.step(a)
-        for x, y, name in zip(r, q, ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=name)
-    rs, os_ = ref.get_state(), orc.get_state()
-    for k in rs:
-        np.testing.assert_array_equal(rs[k], os_[k], err_msg=k)
-    assert (os_["agent"][moved, 3] == 5).sum() >= moved.sum() // 4
+        trace.step(env.step(a), a)
+    st = trace.state(env, full_obs=False)
+    assert (st["agent"][moved, 3] == 5).sum() >= moved.sum() // 4
+
+
+MEMORY_IDS = ["MiniGrid-MemoryS7-v0", "MiniGrid-MemoryS13Random-v0"]
+ROOMGRID_IDS = ["MiniGrid-Unlock-v0", "MiniGrid-UnlockPickup-v0", "MiniGrid-BlockedUnlockPickup-v0", "MiniGrid-KeyCorridorS3R3-v0",
+                "MiniGrid-KeyCorridorS6R3-v0"]
+BOX_IDS = ["MiniGrid-ObstructedMaze-1Dlh-v0", "MiniGrid-ObstructedMaze-Full-v1"]
+
+
+@pytest.mark.parametrize("env_id", MEMORY_IDS)
+def test_memory_success_and_failure_cells_against_live_reference(env_id):
+    replay(f"memory cells {env_id}", memory_cells, env_id)
+
+
+@pytest.mark.parametrize("env_id", ROOMGRID_IDS)
+def test_roomgrid_post_filters_fire_against_live_reference(env_id):
+    replay(f"roomgrid post-filters {env_id}", roomgrid_post_filters, env_id)
+
+
+@pytest.mark.parametrize("env_id", BOX_IDS)
+def test_boxes_hide_keys_against_live_reference(env_id):
+    replay(f"boxes {env_id}", boxes_hide_keys, env_id)

@@ -1,117 +1,98 @@
-"""Live check of the C oracle against the unmodified Python reference (build container only: skipped
-where /root/reference is absent, e.g. on the GPU box)."""
+"""The C oracle against the unmodified Python reference. Every scenario below runs on either side: on the reference's
+own env objects it was recorded once into tests/golden/traces_reference.npz (python -m oracle.gen_golden traces), and
+the tests replay it on the oracle against that recording (oracle/trace.py)."""
+import os
+
 import numpy as np
 import pytest
 
-from oracle import ref_loader
+from oracle import trace as tr
 from oracle.oracle import ENV_SPECS, OracleVecEnv
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not present")
+TRACES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "traces_reference.npz")
+_recorded = None
 
 
-@pytest.mark.parametrize("env_id", list(ENV_SPECS))
-@pytest.mark.parametrize("mode", ["next_step", "same_step"])
-def test_lockstep_rollout(env_id, mode):
-    n, t_steps = 6, 250
-    ref = ref_loader.ReferenceVecEnv(env_id, n, autoreset=mode)
-    orc = OracleVecEnv(env_id, n, autoreset=mode)
-    e0 = ref.envs[0]
-    assert (orc.width, orc.height, orc.max_steps, orc.see_through) == (e0.width, e0.height, e0.max_steps, e0.see_through_walls)
-    ro, rd = ref.reset(seed=1000)
-    oo, od = orc.reset(seed=1000)
-    np.testing.assert_array_equal(ro, oo)
-    np.testing.assert_array_equal(rd, od)
-    rng = np.random.default_rng(77)
+class OracleEnv(OracleVecEnv):
+    """The oracle under the method names oracle.ref_loader.ReferenceVecEnv gives the reference's wrappers."""
+
+    def view_obs(self, view_size):
+        return self.gen_obs_view(view_size)
+
+    def one_hot_obs(self):
+        return self.one_hot(self.obs)
+
+
+def make_oracle(env_id, n, autoreset="next_step", spec=None, gym_kwargs=None, no_death=(), death_cost=-1.0, bonus=None):
+    """The oracle side of a scenario's env maker (gym_kwargs is what the reference's constructor takes instead of spec)."""
+    e = OracleEnv(env_id, n, spec=spec, autoreset=autoreset)
+    if no_death or bonus:
+        e.set_no_death(no_death, death_cost)
+        e.set_bonus(bonus)
+    return e
+
+
+def replay(name, scenario, *args):
+    """Runs scenario(make_oracle, trace, *args) against the recording stored under `name`."""
+    global _recorded
+    if _recorded is None:
+        _recorded = tr.load(TRACES)
+    if name not in _recorded:
+        raise AssertionError(f"no recording of {name}: regenerate the traces (python -m oracle.gen_golden traces)")
+    t = tr.Trace(name, _recorded[name])
+    scenario(make_oracle, t, *args)
+    t.close()
+
+
+# ---- scenarios: make(env_id, n, ...) builds the reference's or the oracle's vector env, trace records or checks ----
+def lockstep(make, trace, env_id, mode, n=6, t_steps=250, seed=1000, action_seed=77, **make_kw):
+    env = make(env_id, n, autoreset=mode, **make_kw)
+    trace.exact("dims", [env.width, env.height, env.max_steps, env.see_through])
+    trace.reset(env.reset(seed=seed))
+    rng = np.random.default_rng(action_seed)
     for t in range(t_steps):
         a = rng.integers(0, 7, n)
-        r = ref.step(a)
-        q = orc.step(a)
-        for x, y, name in zip(r, q, ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=f"{name} t={t}")
-    rs, os_ = ref.get_state(), orc.get_state()
-    for k in rs:
-        np.testing.assert_array_equal(rs[k], os_[k], err_msg=k)
-    np.testing.assert_array_equal(ref.full_obs(), orc.full_obs())
+        trace.step(env.step(a), a)
+    trace.state(env)
 
 
-def test_spec_table_matches_registry():
-    gym, _ = ref_loader.load()
-    for env_id, (kind, w, h, ms, st, prm) in ENV_SPECS.items():
-        e = gym.make(env_id).unwrapped
-        assert (e.width, e.height, e.max_steps, e.see_through_walls) == (w, h, ms, st), env_id
-
-
-@pytest.mark.parametrize("base_id,kind,size,max_steps,see_through,params", [
+UNREGISTERED_SIZES = [
     ("MiniGrid-Empty-5x5-v0", "empty", 26, 4 * 26 * 26, True, [1, 0, 0, 0]),  # agent_start_pos=None: random start
     ("MiniGrid-DoorKey-5x5-v0", "doorkey", 26, 10 * 26 * 26, False, []),
     ("MiniGrid-DoorKey-5x5-v0", "doorkey", 6, 10 * 6 * 6, False, []),
-])
-def test_lockstep_rollout_at_unregistered_sizes(base_id, kind, size, max_steps, see_through, params):
-    """The engine's size limit (26) and a small DoorKey that no id registers: the reference classes take `size`."""
-    n, t_steps = 4, 200
-    kwargs = {"size": size}
+]
+
+
+def unregistered_size(make, trace, base_id, kind, size, max_steps, see_through, params):
+    gym_kwargs = {"size": size}
     if kind == "empty":
-        kwargs["agent_start_pos"] = None
-    ref = ref_loader.ReferenceVecEnv(base_id, n, **kwargs)
-    orc = OracleVecEnv(None, n, spec=(kind, size, size, max_steps, see_through, params))
-    e0 = ref.envs[0]
-    assert (e0.width, e0.height, e0.max_steps, e0.see_through_walls) == (size, size, max_steps, see_through)
-    ro, rd = ref.reset(seed=5)
-    oo, od = orc.reset(seed=5)
-    np.testing.assert_array_equal(ro, oo)
-    np.testing.assert_array_equal(rd, od)
-    rng = np.random.default_rng(6)
-    for t in range(t_steps):
-        a = rng.integers(0, 7, n)
-        for x, y, name in zip(ref.step(a), orc.step(a), ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=f"{name} t={t}")
-    rs, os_ = ref.get_state(), orc.get_state()
-    for k in rs:
-        np.testing.assert_array_equal(rs[k], os_[k], err_msg=k)
+        gym_kwargs["agent_start_pos"] = None
+    lockstep(make, trace, base_id, "next_step", n=4, t_steps=200, seed=5, action_seed=6,
+             spec=(kind, size, size, max_steps, see_through, params), gym_kwargs=gym_kwargs)
 
 
-@pytest.mark.parametrize("env_id", ["MiniGrid-DoorKey-8x8-v0", "MiniGrid-FourRooms-v0", "MiniGrid-Empty-5x5-v0", "MiniGrid-MultiRoom-N6-v0",
-                                    "MiniGrid-Playground-v0", "MiniGrid-Dynamic-Obstacles-6x6-v0"])
-def test_observation_wrappers_against_live_reference(env_id):
-    """SURVEY 8(f-3): ViewSizeWrapper (V = 3, 5, 9, 11), SymbolicObsWrapper and OneHotPartialObsWrapper restated in the
-    oracle (gen_obs_view, symbolic_obs, one_hot) against the reference's own wrapper classes on the same states."""
+WRAPPER_IDS = ["MiniGrid-DoorKey-8x8-v0", "MiniGrid-FourRooms-v0", "MiniGrid-Empty-5x5-v0", "MiniGrid-MultiRoom-N6-v0",
+               "MiniGrid-Playground-v0", "MiniGrid-Dynamic-Obstacles-6x6-v0"]
+
+
+def observation_wrappers(make, trace, env_id):
     n = 6
-    ref = ref_loader.ReferenceVecEnv(env_id, n)
-    orc = OracleVecEnv(env_id, n)
-    ref.reset(seed=31)
-    orc.reset(seed=31)
+    env = make(env_id, n)
+    env.reset(seed=31)
     rng = np.random.default_rng(5)
     for t in range(120):
         a = rng.integers(0, 7, n)
-        r = ref.step(a)
-        q = orc.step(a)
-        np.testing.assert_array_equal(r[0], q[0])
+        trace.step(env.step(a), a)
         if t % 6 == 0:
             for V in (3, 5, 7, 9, 11):
-                np.testing.assert_array_equal(ref.view_obs(V), orc.gen_obs_view(V), err_msg=f"view {V} t={t}")
-            sym = ref.symbolic_obs()
+                trace.digest(f"view {V} t={t}", env.view_obs(V))
+            sym = env.symbolic_obs()
             assert sym.dtype == np.int64
-            np.testing.assert_array_equal(sym, orc.symbolic_obs(), err_msg=f"symbolic t={t}")
-            np.testing.assert_array_equal(ref.one_hot_obs(), OracleVecEnv.one_hot(q[0]), err_msg=f"one-hot t={t}")
+            trace.digest(f"symbolic t={t}", sym)
+            trace.digest(f"one-hot t={t}", env.one_hot_obs())
 
 
-# ---- SURVEY 8(f-4), second half: the reward wrappers (wrappers.py:68-184, 809-882) ----
-def _wrap(no_death, bonus):
-    ref_loader.load()
-    from minigrid.wrappers import ActionBonus, NoDeath, PositionBonus
-
-    def w(e):
-        if no_death:
-            e = NoDeath(e, no_death_types=no_death, death_cost=-1.5)
-        if bonus == "action":
-            e = ActionBonus(e)
-        elif bonus == "position":
-            e = PositionBonus(e)
-        return e
-    return w
-
-
-@pytest.mark.parametrize("env_id,no_death,bonus", [
+REWARD_WRAPPER_CASES = [
     ("MiniGrid-LavaCrossingS9N1-v0", ("lava",), None),
     ("MiniGrid-LavaCrossingS9N3-v0", ("lava",), "action"),
     ("MiniGrid-DistShift1-v0", ("lava",), "position"),
@@ -122,31 +103,60 @@ def _wrap(no_death, bonus):
     ("MiniGrid-DoorKey-5x5-v0", (), "position"),
     ("MiniGrid-FourRooms-v0", (), "action"),
     ("MiniGrid-GoToDoor-5x5-v0", ("door",), "position"),
-])
-@pytest.mark.parametrize("mode", ["next_step", "same_step"])
-def test_reward_wrappers_against_live_reference(env_id, no_death, bonus, mode):
-    """NoDeath, ActionBonus and PositionBonus as a SyncVectorEnv of wrapped envs applies them (bonus outermost), restated
-    in the oracle (wrapped_step): rewards bit for bit, and the episodes NoDeath keeps alive stay alive."""
+]
+
+
+def reward_wrappers(make, trace, env_id, no_death, bonus, mode):
     n, t_steps = 6, 400
-    ref = ref_loader.ReferenceVecEnv(env_id, n, autoreset=mode, wrap=_wrap(no_death, bonus))
-    orc = OracleVecEnv(env_id, n, autoreset=mode)
-    orc.set_no_death(no_death, -1.5)
-    orc.set_bonus(bonus)
-    ref.reset(seed=2)
-    orc.reset(seed=2)
+    env = make(env_id, n, autoreset=mode, no_death=no_death, death_cost=-1.5, bonus=bonus)
+    env.reset(seed=2)
     rng = np.random.default_rng(11)
     saved = 0
     for t in range(t_steps):
         # forward-heavy actions: walk into lava / obstacles often
         a = np.where(rng.random(n) < 0.5, 2, rng.integers(0, 7, n))
-        r = ref.step(a)
-        q = orc.step(a)
-        for x, y, name in zip(r, q, ["obs", "dir", "reward", "terminated", "truncated"]):
-            np.testing.assert_array_equal(np.asarray(x), np.asarray(y), err_msg=f"{name} t={t}")
-        assert r[2].tobytes() == q[2].tobytes()
+        r = trace.step(env.step(a), a)
         saved += int(((r[2] < -0.4) & ~r[3]).sum())  # a negative reward on a live env: the death cost
     if no_death and "Empty" not in env_id and "GoToDoor" not in env_id:
         assert saved > 0, "NoDeath never triggered: the test does not cover it"
+
+
+# ---- tests ----
+@pytest.mark.parametrize("env_id", list(ENV_SPECS))
+@pytest.mark.parametrize("mode", ["next_step", "same_step"])
+def test_lockstep_rollout(env_id, mode):
+    replay(f"lockstep {env_id} {mode}", lockstep, env_id, mode)
+
+
+def test_spec_table_matches_registry():
+    """(width, height, max_steps, see_through_walls) of gym.make(id).unwrapped, recorded for every id of ENV_SPECS."""
+    def check(make, trace):
+        for env_id, spec in ENV_SPECS.items():
+            trace.exact(env_id, list(spec[1:5]))
+
+    replay("registry", check)
+
+
+@pytest.mark.parametrize("base_id,kind,size,max_steps,see_through,params", UNREGISTERED_SIZES)
+def test_lockstep_rollout_at_unregistered_sizes(base_id, kind, size, max_steps, see_through, params):
+    """The engine's size limit (26) and a small DoorKey that no id registers: the reference classes take `size`."""
+    replay(f"unregistered {base_id} {size}", unregistered_size, base_id, kind, size, max_steps, see_through, params)
+
+
+@pytest.mark.parametrize("env_id", WRAPPER_IDS)
+def test_observation_wrappers_against_live_reference(env_id):
+    """SURVEY 8(f-3): ViewSizeWrapper (V = 3, 5, 9, 11), SymbolicObsWrapper and OneHotPartialObsWrapper restated in the
+    oracle (gen_obs_view, symbolic_obs, one_hot) against the reference's own wrapper classes on the same states."""
+    replay(f"observation wrappers {env_id}", observation_wrappers, env_id)
+
+
+# ---- SURVEY 8(f-4), second half: the reward wrappers (wrappers.py:68-184, 809-882) ----
+@pytest.mark.parametrize("env_id,no_death,bonus", REWARD_WRAPPER_CASES)
+@pytest.mark.parametrize("mode", ["next_step", "same_step"])
+def test_reward_wrappers_against_live_reference(env_id, no_death, bonus, mode):
+    """NoDeath, ActionBonus and PositionBonus as a SyncVectorEnv of wrapped envs applies them (bonus outermost), restated
+    in the oracle (wrapped_step): rewards bit for bit, and the episodes NoDeath keeps alive stay alive."""
+    replay(f"reward wrappers {env_id} {mode}", reward_wrappers, env_id, no_death, bonus, mode)
 
 
 def test_reward_wrapper_known_answers():
@@ -166,24 +176,25 @@ def test_reward_wrapper_known_answers():
     r = o.step([2]); assert (float(r[2][0]), bool(r[3][0])) == (-2.0, False)
 
 
+def constant_mission_ids():
+    from minigrid_b200 import specs
+
+    return [env_id for env_id in (specs.all_ids() if hasattr(specs, "all_ids") else list(ENV_SPECS))
+            if "{" not in specs.get(env_id).mission]
+
+
 def test_dict_observation_space_wrapper_mission_indices():
     """minigrid_b200.wrappers.mission_to_indices against the reference's DictObservationSpaceWrapper (wrappers.py:428-554) on the
-    constant mission strings of the registered ids (its doctest value included: LavaCrossingS11N5 -> [19, 31, 17, 36, 20, 38, ...])."""
-    gym, _ = ref_loader.load()
-    from minigrid.wrappers import DictObservationSpaceWrapper as RefDict
-
+    constant mission strings of the registered ids (its doctest value included: LavaCrossingS11N5 -> [19, 31, 17, 36, 20, 38, ...]).
+    The recording holds the wrapper's word list (get_minigrid_words, in index order) and obs["mission"] after reset(seed=0)."""
     from minigrid_b200 import specs
     from minigrid_b200.wrappers import MINIGRID_WORDS, mission_to_indices
 
-    assert {w: i for i, w in enumerate(MINIGRID_WORDS)} == RefDict.get_minigrid_words()
-    seen = 0
-    for env_id in specs.all_ids() if hasattr(specs, "all_ids") else list(ENV_SPECS):
-        mission = specs.get(env_id).mission
-        if "{" in mission:
-            continue
-        e = RefDict(gym.make(env_id))
-        obs, _ = e.reset(seed=0)
-        assert obs["mission"] == mission_to_indices(mission), env_id
-        seen += 1
-    assert seen >= 20
+    def check(make, trace):
+        trace.exact("words", list(MINIGRID_WORDS))
+        for env_id in constant_mission_ids():
+            trace.exact(f"mission {env_id}", mission_to_indices(specs.get(env_id).mission))
+
+    replay("dict observation", check)
+    assert len(constant_mission_ids()) >= 20
     assert mission_to_indices("avoid the lava and get to the green goal square")[:10] == [19, 31, 17, 36, 20, 38, 31, 2, 15, 35]
