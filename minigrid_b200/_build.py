@@ -9,7 +9,7 @@ import subprocess
 _PKG = os.path.dirname(os.path.abspath(__file__))
 _CSRC = os.path.join(_PKG, "csrc")
 LIB_PATH = os.path.join(_PKG, "libminigrid_b200.so")
-SOURCES = ["mg_abi.cu", "mg_step.cu", "mg_step_tiled1.cu", "mg_step_window.cu", "mg_reset.cu", "mg_state.cu", "mg_wrappers.cu", "mg_host_expand.cpp"]
+SOURCES = ["mg_abi.cu", "mg_step.cu", "mg_step_window.cu", "mg_reset.cu", "mg_state.cu", "mg_wrappers.cu", "mg_host_expand.cpp"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--threads", "0"]
 

@@ -186,11 +186,8 @@ int mg_create(int kind, int width, int height, int max_steps, int see_through_wa
   p.mode = autoreset_mode;
   p.kind = kind;
   h->trace = getenv("MINIGRID_B200_HOST_TRACE") != nullptr;
-  { const char *wp = getenv("MINIGRID_B200_WINPREF"); h->p.win_prefetch = !wp || atoi(wp) != 0; }
   h->stream_fixed = -1;
   if (const char *es = getenv("MINIGRID_B200_EXPAND_STREAM")) h->stream_fixed = atoi(es) != 0;
-  p.hot_first = 1;
-  if (const char *e = getenv("MINIGRID_B200_HOTFIRST")) p.hot_first = atoi(e) != 0;  // tuning knob (same-box A/B)
   for (int i = 0; i < 8; ++i) p.kp[i] = (params && i < n_params) ? params[i] : 0;
   if (kind == MG_KIND_EMPTY && !p.kp[0] && n_params < 4) { p.kp[1] = 1; p.kp[2] = 1; p.kp[3] = 0; }
   if (kind == MG_KIND_CROSSING && n_params < 2) { p.kp[0] = 1; p.kp[1] = (int)T_LAVA; }
@@ -267,8 +264,8 @@ int mg_create(int kind, int width, int height, int max_steps, int see_through_wa
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_order, cudaEventDisableTiming);
   if (e == cudaSuccess) e = configure_step(p, &h->plan);
   if (e == cudaSuccess && getenv("MINIGRID_B200_VERBOSE"))
-    fprintf(stderr, "[minigrid_b200] K1 plan: layout=%d, %d warps/CTA, vis=%d, nbuf=%d, %d CTA/SM, grid=%d, smem=%zu B, tiles=%d\n", p.g.layout, h->plan.warps,
-            h->plan.vis, h->plan.nbuf, h->plan.ctas_per_sm, h->plan.grid, h->plan.smem, p.n_tiles);
+    fprintf(stderr, "[minigrid_b200] K1 plan: layout=%d, %d warps/CTA, vis=%d, %d CTA/SM, grid=%d, smem=%zu B, tiles=%d\n", p.g.layout, h->plan.warps,
+            h->plan.vis, h->plan.ctas_per_sm, h->plan.grid, h->plan.smem, p.n_tiles);
   if (e == cudaSuccess) e = launch_init(p, h->hstream);
   if (e == cudaSuccess) e = launch_template(p, d_tm, h->hstream);
   if (e == cudaSuccess) e = launch_seed(p, nullptr, nullptr, 0, h->hstream);

@@ -162,9 +162,7 @@ struct Params {
   const uint16_t *vis_tbl;  // [128 * 128] process_vis row table (mg_obs.cuh: build_vis_table)
   const uint32_t *tmpl;     // [wpe] level template: the words of a blank draw (mg_levels.cuh)
   int *err;                 // sticky error word
-  int hot_first;            // visit the tiles flagged in tile_hot right after a CTA's first round (MINIGRID_B200_HOTFIRST=0 turns it off)
   uint8_t *tile_hot;        // [n_tiles] 1 = an env of the tile ended in the last step (K1's scheduling hint, never semantics)
-  int win_prefetch;         // LAYOUT_WINDOW: L2-prefetch the next tile's view lines (MINIGRID_B200_WINPREF=0 turns it off)
   // the reference's reward wrappers around every env (wrappers.py:68-184, 809-882), 0 = absent
   int no_death_mask;        // NoDeath: bit t = OBJECT_TO_IDX type t is a death cell
   int bonus_mode;           // 1 ActionBonus, 2 PositionBonus
@@ -173,7 +171,7 @@ struct Params {
 };
 
 struct StepPlan {  // launch shape of K1, chosen once per handle (mg_step.cu: configure_step)
-  int warps, vis, nbuf, mode, ctas_per_sm, grid;
+  int warps, vis, ctas_per_sm, grid;
   size_t smem;
 };
 

@@ -4,9 +4,8 @@
 // One warp = one tile of 32 environments, one lane per environment.
 //   1. lane 0 issues a TMA bulk copy (cp.async.bulk -> SASS UBLKCP) of the tile's interleaved grid words
 //      into shared memory and arms an mbarrier with the byte count; meanwhile every lane loads its
-//      action and 16-byte agent record with coalesced loads. Warps are persistent (one CTA per SM, one wave). Default
-//      plan: one buffer per warp, 22 warps at 72 registers (mg_step_tiled1.cu); the two-buffer form, in which a warp
-//      requests its next tile (copy + records + actions) while it works on the current one, is this file's (configure_step).
+//      action and 16-byte agent record with coalesced loads. Warps are persistent (one CTA per SM, one wave): one
+//      buffer per warp, 22 warps at 72 registers (configure_step).
 //   2. autoreset (NEXT_STEP: envs flagged last step, before the transition; SAME_STEP: envs that just ended,
 //      after it): rare; the pending lanes replay their env's numpy-exact RNG draws while the idle lanes copy the level
 //      template over those envs, then the warp patches the few draw-dependent cells (warp_reset).
@@ -17,85 +16,56 @@
 //   5. coalesced stores of direction / reward / terminated / truncated and the agent record.
 // Large grids (LAYOUT_WINDOW) skip step 1: each lane gathers only the 7 lines its view needs straight into registers
 // (21 independent 4-byte loads, one round trip; mg_obs.cuh: load_view_words), and the transition reads its front cell
-// out of the same words.
+// out of the same words. This file holds the tiled instantiations, mg_step_window.cu the window ones.
 #include "mg_step_kernel.cuh"
 
 namespace mg {
 
 #ifdef MG_TIMELINE
 int debug_timeline_window(void *out);
-int debug_timeline_tiled1(void *out);
-extern "C" int mg_debug_timeline(void *out, int mode) {  // out: unsigned long long[2][160][16]; mode: MODE_* of the handle's plan
-  if (mode == MODE_WINDOW) return debug_timeline_window(out);
-  if (mode == MODE_TILED1) return debug_timeline_tiled1(out);
+extern "C" int mg_debug_timeline(void *out, int layout) {  // out: unsigned long long[2][160][16]; layout: LAYOUT_* of the handle
+  if (layout == LAYOUT_WINDOW) return debug_timeline_window(out);
   return (int)cudaMemcpyFromSymbol(out, g_tl, sizeof(g_tl));
 }
 #endif
 
-static StepKernel step_kernel(int kind, int vis, int mode) {
-  if (mode == MODE_WINDOW) return step_kernel_window(kind, vis);
-  return mode == MODE_TILED2 ? pick_vis<MODE_TILED2>(kind, vis) : step_kernel_tiled1(kind, vis);
+static StepKernel step_kernel(int kind, int vis, int layout) {
+  return layout == LAYOUT_WINDOW ? step_kernel_window(kind, vis) : pick_vis<LAYOUT_TILED>(kind, vis);
 }
 
-// Choose the CTA shape once per handle: one persistent CTA per SM. Measured preferences on the final kernels
-// (profiles/r02o..r02q_gpu_call.log, 262144 envs, desynchronised episodes): for the tiled layout the ONE-buffer kernel
-// at 72 registers with about 22 warps beats the two-buffer kernel at 96 registers with 19 on every kind tried (DoorKey
-// 18.8 against 21.5 us, Empty 18.5 / 19.6, GoToDoor 125 / 157, Fetch 30.4 / 36.8; 20..22 warps is a plateau, 24..28 a
-// little behind, 16 clearly) — round 1's "prefetching beats occupancy" no longer holds now that regenerating tiles go
-// first and the tile loop is shorter; the table-driven process_vis (32 KB of shared memory) beats the ALU form; the
-// window layout wants all 20 warps its 96 registers allow (at 72 registers and 28 warps it spills and loses).
-// MINIGRID_B200_CFG="warps,vis,nbuf" (vis: 1 ALU, 2 table) overrides the choice (tuning knob).
+// Choose the CTA shape once per handle: one persistent CTA per SM. Measured on the final kernels
+// (profiles/r02o..r02q_gpu_call.log, 262144 envs, desynchronised episodes): the tiled kernel at 72 registers wants about
+// 22 warps (20..22 is a plateau, 24..28 a little behind, 16 clearly), the window kernel all 20 warps its 96 registers
+// allow (at 72 registers and 28 warps it spills and loses), and the table-driven process_vis (32 KB of shared memory)
+// beats the ALU form. MINIGRID_B200_CFG="warps" overrides the warp count (tuning and test knob).
 cudaError_t configure_step(const Params &p, StepPlan *plan) {
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  int want_warps = 0, want_vis = 0, want_nbuf = 0;
-  if (const char *cfg = getenv("MINIGRID_B200_CFG")) sscanf(cfg, "%d,%d,%d", &want_warps, &want_vis, &want_nbuf);
+  int want_warps = 0;
+  if (const char *cfg = getenv("MINIGRID_B200_CFG")) sscanf(cfg, "%d", &want_warps);
   const bool win = p.g.layout == LAYOUT_WINDOW;
-  double best_score = -1.0;
-  plan->warps = 0;
-  const int vis_opts[2] = {VIS_TBL, VIS_ALU};
-  for (int vi = 0; vi < (p.see_through ? 1 : 2); ++vi) {
-    const int vis = p.see_through ? VIS_NONE : vis_opts[vi];
-    if (!p.see_through && want_vis && vis != want_vis) continue;
-    for (int nbuf = win ? 1 : 2; nbuf >= 1; --nbuf) {
-      if (!win && want_nbuf && nbuf != want_nbuf) continue;
-      const int mode = win ? MODE_WINDOW : (nbuf == 2 ? MODE_TILED2 : MODE_TILED1);
-      StepKernel k = step_kernel(p.kind, vis, mode);
-      const int wcap = (nbuf == 2 || win) ? 20 : 28;  // __launch_bounds__ of the variants
-      int wmax = 0;
-      for (int w = wcap; w >= 1; --w)
-        if (step_smem_bytes(p.g, vis, w, nbuf) <= 227 * 1024 - 1024) { wmax = w; break; }
-      if (wmax == 0) continue;
-      cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)step_smem_bytes(p.g, vis, wmax, nbuf));
-      if (e != cudaSuccess) return e;
-      for (int w = wmax; w >= (want_warps ? 1 : (wmax + 1) / 2); --w) {
-        if (want_warps && w != want_warps) continue;
-        const size_t smem = step_smem_bytes(p.g, vis, w, nbuf);
-        int ctas = 0;
-        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, k, w * 32, smem);
-        if (e != cudaSuccess) return e;
-        if (ctas < 1) continue;
-        if (ctas * w > wcap) ctas = wcap / w;
-        if (ctas < 1) continue;
-        const int resident = ctas * w;
-        const int target = win ? 20 : (nbuf == 1 ? 22 : 14);  // see above
-        const int off = resident > target ? resident - target : target - resident;
-        const double score = (win || nbuf == 1 ? 2.0 : 1.0) * (vis == VIS_TBL ? 1.3 : 1.0) - 0.02 * off;
-        if (score > best_score + 1e-9) {
-          best_score = score;
-          plan->warps = w; plan->vis = vis; plan->nbuf = nbuf; plan->mode = mode; plan->ctas_per_sm = ctas; plan->smem = smem;
-        }
-      }
-    }
-  }
-  if (plan->warps == 0) return cudaErrorInvalidValue;
+  const int vis = p.see_through ? VIS_NONE : VIS_TBL;
+  const int wcap = win ? 20 : 28;  // __launch_bounds__ of the kernel
+  int wmax = wcap;  // the most warps whose buffers fit
+  while (wmax >= 1 && step_smem_bytes(p.g, vis, wmax) > 227 * 1024 - 1024) --wmax;
+  const int w = want_warps ? want_warps : min(win ? 20 : 22, wmax);
+  if (w < 1 || w > wmax) return cudaErrorInvalidValue;
+  StepKernel k = step_kernel(p.kind, vis, p.g.layout);
+  cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)step_smem_bytes(p.g, vis, wmax));
+  if (e != cudaSuccess) return e;
+  const size_t smem = step_smem_bytes(p.g, vis, w);
+  int ctas = 0;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, k, w * 32, smem);
+  if (e != cudaSuccess) return e;
+  if (ctas * w > wcap) ctas = wcap / w;
+  if (ctas < 1) return cudaErrorInvalidValue;
+  plan->warps = w; plan->vis = vis; plan->ctas_per_sm = ctas; plan->smem = smem;
   const long long want = ((long long)p.n_tiles + plan->warps - 1) / plan->warps;
   long long grid = (long long)sms * plan->ctas_per_sm;
   if (grid > want) grid = want;
   // test knob: fewer CTAs than the device offers, so that a SMALL batch gives every warp several tiles (the tile loop's
-  // prefetch / buffer rotation / order list are otherwise only exercised at BASELINE sizes)
+  // prefetch / order list are otherwise only exercised at BASELINE sizes)
   if (const char *e = getenv("MINIGRID_B200_GRID")) { const long long cap = atoll(e); if (cap >= 1 && cap < grid) grid = cap; }
   plan->grid = (int)(grid < 1 ? 1 : grid);
   return cudaSuccess;
@@ -110,8 +80,7 @@ cudaError_t launch_step(const Params &p, const StepPlan &plan, const void *actio
   static int launch_no = 0;
   tma_ok |= (launch_no++ & 1) << 1;
 #endif
-  StepKernel k = step_kernel(p.kind, plan.vis, plan.mode);
-  static const bool use_pdl = []() { const char *e = getenv("MINIGRID_B200_PDL"); return !e || atoi(e) != 0; }();
+  StepKernel k = step_kernel(p.kind, plan.vis, p.g.layout);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)plan.grid);
   cfg.blockDim = dim3((unsigned)plan.warps * 32);
@@ -121,7 +90,7 @@ cudaError_t launch_step(const Params &p, const StepPlan &plan, const void *actio
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = use_pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, k, p, actions, action_dtype, obs, dir, reward, term, trunc, packed, tma_ok);
 }
 

@@ -1,6 +1,5 @@
-// mg_step_kernel.cuh — K1, the step kernel template (see mg_step.cu for the overview). It is instantiated in three
-// translation units, mg_step.cu (tiled layout, two buffers per warp), mg_step_tiled1.cu (one buffer: the default plan) and
-// mg_step_window.cu (window layout): ptxas's code for the tiled
+// mg_step_kernel.cuh — K1, the step kernel template (see mg_step.cu for the overview). It is instantiated in two
+// translation units, mg_step.cu (tiled layout) and mg_step_window.cu (window layout): ptxas's code for the tiled
 // kernels measurably depends on what else it compiles alongside them (profiles/README.md, r01 A/B runs).
 #pragma once
 #include <cstdio>
@@ -15,10 +14,8 @@
 
 namespace mg {
 
-enum : int { MODE_TILED1 = 0, MODE_TILED2 = 1, MODE_WINDOW = 2 };  // buffers per warp / layout of K1
-
 #ifdef MG_TIMELINE  // debug build only (scripts/timeline.py): per-CTA %globaltimer stamps of the last two launches
-static __device__ unsigned long long g_tl[2][160][16];  // one per translation unit: mg_debug_timeline(mode) reads the right one
+static __device__ unsigned long long g_tl[2][160][16];  // one per translation unit: mg_debug_timeline(layout) reads the right one
 //  // 0-7: CTA stamps; 8: regenerating tiles, 9 / 10: longest regenerating / plain tile (ns), 11: end of the last regenerating tile, 12: its pull index, 13: list ready
 __device__ __forceinline__ unsigned long long gtime() {
   unsigned long long t;
@@ -47,9 +44,9 @@ __host__ __device__ inline uint32_t step_buf_bytes(const Geom &g) {
 // front. The list is built in the prologue, i.e. before griddepcontrol.wait, from flags the previous launch may still
 // be writing: a stale flag only costs the tile its place in the order, never correctness.
 constexpr int ORDER_CAP = 1024;
-// [cell table 1 KB][visibility table 32 KB, VIS_TBL only][warps x nbuf x buffer][mbarriers][tile counter][list barrier][order list]
-__host__ __device__ inline size_t step_smem_bytes(const Geom &g, int vis, int warps, int nbuf) {
-  return 1024 + (vis == VIS_TBL ? VIS_TBL_BYTES : 0) + (size_t)warps * nbuf * step_buf_bytes(g) + 16 * (size_t)warps + 32 + 2 * ORDER_CAP;
+// [cell table 1 KB][visibility table 32 KB, VIS_TBL only][warps x buffer][warps x mbarrier][table mbarrier][tile counter][order list]
+__host__ __device__ inline size_t step_smem_bytes(const Geom &g, int vis, int warps) {
+  return 1024 + (vis == VIS_TBL ? VIS_TBL_BYTES : 0) + (size_t)warps * step_buf_bytes(g) + 8 * (size_t)warps + 32 + 2 * ORDER_CAP;
 }
 
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
@@ -256,19 +253,17 @@ __device__ __noinline__ ResetOut warp_reset(const Params &p, unsigned pend, int 
   return out;
 }
 
-// MODE_TILED2: each warp owns two buffers and prefetches its next tile (TMA + agent records + actions) before it
-// processes the current one, so HBM transfers overlap compute instead of alternating with it in GPU-wide bursts.
-template <int KIND, int VIS, int MODE>
-__global__ void __launch_bounds__(MODE == MODE_TILED2 ? 640 : (MODE == MODE_TILED1 ? 896 : 640), 1)  // one CTA per SM: <= 20 warps (96 regs; the window mode keeps 21 view words live) or <= 28 (72 regs: 7 warps per scheduler)
+// LAYOUT_TILED: each warp stages its tile in one shared-memory buffer by a bulk copy. LAYOUT_WINDOW: each lane loads
+// its view window into registers, and the warp fetches the next tile's agent records and actions one tile ahead.
+template <int KIND, int VIS, int LAYOUT>
+__global__ void __launch_bounds__(LAYOUT == LAYOUT_TILED ? 896 : 640, 1)  // one CTA per SM: tiled <= 28 warps (72 regs: 7 warps per scheduler), window <= 20 (96 regs: it keeps 21 view words live)
 k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int act_dtype, uint8_t *__restrict__ obs,
        int32_t *__restrict__ dir_out, double *__restrict__ reward_out, uint8_t *__restrict__ term_out,
        uint8_t *__restrict__ trunc_out, uint32_t *__restrict__ packed_out, int obs_tma_ok) {
-  constexpr int NBUF = (MODE == MODE_TILED2) ? 2 : 1;
-  constexpr bool WIN = (MODE == MODE_WINDOW);
-  constexpr bool PREF = (MODE != MODE_TILED1);  // agent records / actions / tile index are fetched one tile ahead
+  constexpr bool WIN = (LAYOUT == LAYOUT_WINDOW);  // agent records / actions / tile index are fetched one tile ahead
   extern __shared__ __align__(128) uint8_t smem_raw[];
   Geom g = p.g;
-  g.layout = WIN ? LAYOUT_WINDOW : LAYOUT_TILED;  // both are implied by MODE: let the compiler fold them
+  g.layout = LAYOUT;  // both are implied by LAYOUT: let the compiler fold them
   g.ring = WIN ? 3 : 1;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int WARPS = blockDim.x >> 5;
@@ -278,11 +273,11 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
 
   uint32_t *lut = reinterpret_cast<uint32_t *>(smem_raw);
   const uint16_t *vis_tbl = reinterpret_cast<const uint16_t *>(smem_raw + 1024);
-  uint8_t *bufs = smem_raw + 1024 + TBL + (size_t)warp * NBUF * buf_bytes;
-  uint64_t *bars = reinterpret_cast<uint64_t *>(smem_raw + 1024 + TBL + (size_t)WARPS * NBUF * buf_bytes);
-  const uint32_t bar0 = smem_u32(bars + 2 * warp), tbl_bar = smem_u32(bars + 2 * WARPS);
-  int *s_next = reinterpret_cast<int *>(bars + 2 * WARPS + 1);
-  uint16_t *s_order = reinterpret_cast<uint16_t *>(bars + 2 * WARPS + 3);
+  uint32_t *gtile = reinterpret_cast<uint32_t *>(smem_raw + 1024 + TBL + (size_t)warp * buf_bytes);
+  uint64_t *bars = reinterpret_cast<uint64_t *>(smem_raw + 1024 + TBL + (size_t)WARPS * buf_bytes);
+  const uint32_t bar = smem_u32(bars + warp), tbl_bar = smem_u32(bars + WARPS);
+  int *s_next = reinterpret_cast<int *>(bars + WARPS + 1);
+  uint16_t *s_order = reinterpret_cast<uint16_t *>(bars + WARPS + 3);
 
   // Programmatic dependent launch: let the next kernel in the stream start its prologue while this grid drains,
   // and do our own prologue (nothing the previous step wrote is touched) before waiting for it to complete.
@@ -303,9 +298,9 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
   // pull index k of a CTA: its k-th tile. k < WARPS: the static first round; behind it, the order list (flagged tiles first)
   const int n_my = t_hi - t_lo;
   const int m_ord = min(n_my, ORDER_CAP);
-  const bool use_order = stepping && p.mode == AUTORESET_NEXT_STEP && p.hot_first && m_ord > WARPS;
+  const bool use_order = stepping && p.mode == AUTORESET_NEXT_STEP && m_ord > WARPS;
   if (threadIdx.x == 0) {
-    *s_next = (PREF ? 2 : 1) * WARPS;
+    *s_next = (WIN ? 2 : 1) * WARPS;
     if (VIS == VIS_TBL) {  // the table is immutable after mg_create: its copy may run ahead of griddepcontrol.wait
       mbar_init(tbl_bar, 1);
       asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -354,8 +349,7 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
     }
   }
   if (lane == 0) {
-    mbar_init(bar0, 1);
-    mbar_init(bar0 + 8, 1);
+    mbar_init(bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   // the 256-entry (type, colour, state) table is pure arithmetic: no global load anywhere near the critical path
@@ -366,57 +360,36 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
   MG_TL(2);
   bool first = true;  // first tile of this warp
   int tile = map_tile(warp);
-  int next = PREF ? map_tile(WARPS + warp) : p.n_tiles;
+  int next = WIN ? map_tile(WARPS + warp) : p.n_tiles;
 
   uint4 rec = make_uint4(0, 0, 0, 0);
   int action = A_DONE;
-  if (PREF && tile < p.n_tiles) {
-    if (NBUF == 2 && lane == 0) {
-      mbar_expect_tx(bar0, tile_bytes);
-      tma_load_1d(smem_u32(bufs), p.grid + (size_t)tile * g.wpe * 32, tile_bytes, bar0);
-    }
+  if (WIN && tile < p.n_tiles) {
     const int env0 = tile * TILE + lane;
     rec = ldg_rec(p.agent + env0);
     if (stepping && env0 < p.n_envs) action = load_action(actions, act_dtype, env0);
-    // an env that regenerates in this step starts from its RNG record: bring it in while the tile is on its way
+    // an env that regenerates in this step starts from its RNG record: bring it in early
     if (stepping && ((rec.y >> 8) & FLAG_PENDING)) prefetch_rng(p.rng + env0);
   }
 
   uint8_t *gb = reinterpret_cast<uint8_t *>(p.grid);
-  uint32_t phase = 0;  // bit b = parity to wait for on buffer b
-  int b = 0;
+  uint32_t phase = 0;  // parity to wait for on the warp's mbarrier
   while (tile < p.n_tiles) {
     uint4 rec_n = make_uint4(0, 0, 0, 0);
     int action_n = A_DONE, nn = p.n_tiles;
-    // prefetch the next tile (into the other buffer), its agent records and actions, and the index of the tile after it
-    auto prefetch = [&]() {
-      if (next < p.n_tiles) {
-        if (lane == 0) {
-          if (NBUF == 2) {
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the obs block staged there two tiles ago
-            const uint32_t nb = bar0 + 8u * (uint32_t)(b ^ 1);
-            mbar_expect_tx(nb, tile_bytes);
-            tma_load_1d(smem_u32(bufs + (size_t)(b ^ 1) * buf_bytes), p.grid + (size_t)next * g.wpe * 32, tile_bytes, nb);
-          }
-          nn = map_tile(atomicAdd(s_next, 1));  // shared-memory atomic, consumed one tile later
-        }
+    if (WIN) {
+      if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the previous obs block has left
+      if (next < p.n_tiles) {  // the next tile's agent records and actions, and the index of the tile after it
+        if (lane == 0) nn = map_tile(atomicAdd(s_next, 1));  // shared-memory atomic, consumed one tile later
         const int env_n = next * TILE + lane;
         rec_n = ldg_rec(p.agent + env_n);
         if (stepping && env_n < p.n_envs) action_n = load_action(actions, act_dtype, env_n);
       }
-    };
-    // A warp's first tile: every warp of the GPU is fetching its first tile at this moment, and nothing can be
-    // computed anywhere until those arrive, so the second tile is requested only once the first is here (its fetch
-    // then overlaps the first tile's compute like every later one) instead of doubling the opening burst.
-    const bool defer = (NBUF == 2) && first;
-    if (PREF) {
-      if (WIN && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the previous obs block has left
-      if (!defer) prefetch();
     } else {
       if (lane == 0) {
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // the previous obs block has left the buffer
-        mbar_expect_tx(bar0, tile_bytes);
-        tma_load_1d(smem_u32(bufs), p.grid + (size_t)tile * g.wpe * 32, tile_bytes, bar0);
+        mbar_expect_tx(bar, tile_bytes);
+        tma_load_1d(smem_u32(gtile), p.grid + (size_t)tile * g.wpe * 32, tile_bytes, bar);
       }
       const int env0 = tile * TILE + lane;
       rec = ldg_rec(p.agent + env0);
@@ -424,13 +397,12 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
       if (stepping && ((rec.y >> 8) & FLAG_PENDING)) prefetch_rng(p.rng + env0);
       // (Pulling the next tile's index here and asking L2 for its block a tile ahead was measured and rejected: DoorKey
       // 18.8 -> 20.2 us, Fetch 30.5 -> 34.1: committing a warp to its next tile one tile early costs more balance than
-      // the shorter copy wins, profiles/r02w_gpu_call.log. The same early commitment is what the two-buffer kernel pays.)
+      // the shorter copy wins, profiles/r02w_gpu_call.log.)
     }
 #ifdef MG_TIMELINE
     const unsigned long long tl_t0 = gtime();
     bool tl_hot = false;
 #endif
-    uint32_t *gtile = reinterpret_cast<uint32_t *>(bufs + (size_t)b * buf_bytes);
     const int env = tile * TILE + lane;
     const bool active = env < p.n_envs;
     int ax = rec.x & 0xFF, ay = (rec.x >> 8) & 0xFF;
@@ -442,12 +414,11 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
     int tx = PF ? (int)((rec.x >> 16) & 0xFFu) : 0, ty = PF ? (int)(rec.x >> 24) : 0;
 
     if (!WIN) {
-      mbar_wait(bar0 + 8u * (uint32_t)b, (phase >> b) & 1u);
-      phase ^= 1u << b;
+      mbar_wait(bar, phase);
+      phase ^= 1u;
 #ifdef MG_TIMELINE
       if (first) MG_TL(3);
 #endif
-      if (defer) prefetch();
     } else {
       __syncwarp();  // lane 0 has waited for the bulk store that was still reading this buffer
     }
@@ -630,7 +601,7 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
     // this tile, have arrived by now: ask L2 for the 7 lines that tile's gather will read (contiguous: 7 * lsw words),
     // so that the gather finds them a few hundred cycles away instead of in HBM. Hints only: a lane that regenerates
     // its env in the next tile prefetches lines it will not use.
-    if (WIN && PREF && p.win_prefetch && next < p.n_tiles) {
+    if (WIN && next < p.n_tiles) {
       const int axn = rec_n.x & 0xFF, ayn = (rec_n.x >> 8) & 0xFF, dn0 = rec_n.y & 3;
       const int dnn = stepping ? ((dn0 + (action_n == A_LEFT ? 3 : 0) + (action_n == A_RIGHT ? 1 : 0)) & 3) : dn0;
       const bool useCn = dnn & 1;
@@ -735,13 +706,12 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
     }
 #endif
     first = false;
-    if (PREF) {
+    if (WIN) {
       if (stepping && next < p.n_tiles && ((rec_n.y >> 8) & FLAG_PENDING)) prefetch_rng(p.rng + (size_t)next * TILE + lane);
       tile = next;
       next = __shfl_sync(0xFFFFFFFFu, nn, 0);
       rec = rec_n;
       action = action_n;
-      if (NBUF == 2) b ^= 1;
     } else {
       if (lane == 0) nn = map_tile(atomicAdd(s_next, 1));
       tile = __shfl_sync(0xFFFFFFFFu, nn, 0);
@@ -758,36 +728,33 @@ k_step(const __grid_constant__ Params p, const void *__restrict__ actions, int a
 
 typedef void (*StepKernel)(Params, const void *, int, uint8_t *, int32_t *, double *, uint8_t *, uint8_t *, uint32_t *, int);
 
-template <int VIS, int MODE>
+template <int VIS, int LAYOUT>
 static StepKernel pick_kind(int kind) {
   switch (kind) {
-    case KIND_EMPTY: return (StepKernel)k_step<KIND_EMPTY, VIS, MODE>;
-    case KIND_DOORKEY: return (StepKernel)k_step<KIND_DOORKEY, VIS, MODE>;
-    case KIND_CROSSING: return (StepKernel)k_step<KIND_CROSSING, VIS, MODE>;
-    case KIND_LAVAGAP: return (StepKernel)k_step<KIND_LAVAGAP, VIS, MODE>;
-    case KIND_DISTSHIFT: return (StepKernel)k_step<KIND_DISTSHIFT, VIS, MODE>;
-    case KIND_MULTIROOM: return (StepKernel)k_step<KIND_MULTIROOM, VIS, MODE>;
-    case KIND_LOCKEDROOM: return (StepKernel)k_step<KIND_LOCKEDROOM, VIS, MODE>;
-    case KIND_PLAYGROUND: return (StepKernel)k_step<KIND_PLAYGROUND, VIS, MODE>;
-    case KIND_GOTODOOR: return (StepKernel)k_step<KIND_GOTODOOR, VIS, MODE>;
-    case KIND_FETCH: return (StepKernel)k_step<KIND_FETCH, VIS, MODE>;
-    case KIND_REDBLUEDOORS: return (StepKernel)k_step<KIND_REDBLUEDOORS, VIS, MODE>;
-    case KIND_GOTOOBJECT: return (StepKernel)k_step<KIND_GOTOOBJECT, VIS, MODE>;
-    case KIND_PUTNEAR: return (StepKernel)k_step<KIND_PUTNEAR, VIS, MODE>;
-    case KIND_MEMORY: return (StepKernel)k_step<KIND_MEMORY, VIS, MODE>;
-    case KIND_DYNOBS: return (StepKernel)k_step<KIND_DYNOBS, VIS, MODE>;
-    case KIND_ROOMGRID: return (StepKernel)k_step<KIND_ROOMGRID, VIS, MODE>;
-    default: return (StepKernel)k_step<KIND_FOURROOMS, VIS, MODE>;
+    case KIND_EMPTY: return (StepKernel)k_step<KIND_EMPTY, VIS, LAYOUT>;
+    case KIND_DOORKEY: return (StepKernel)k_step<KIND_DOORKEY, VIS, LAYOUT>;
+    case KIND_CROSSING: return (StepKernel)k_step<KIND_CROSSING, VIS, LAYOUT>;
+    case KIND_LAVAGAP: return (StepKernel)k_step<KIND_LAVAGAP, VIS, LAYOUT>;
+    case KIND_DISTSHIFT: return (StepKernel)k_step<KIND_DISTSHIFT, VIS, LAYOUT>;
+    case KIND_MULTIROOM: return (StepKernel)k_step<KIND_MULTIROOM, VIS, LAYOUT>;
+    case KIND_LOCKEDROOM: return (StepKernel)k_step<KIND_LOCKEDROOM, VIS, LAYOUT>;
+    case KIND_PLAYGROUND: return (StepKernel)k_step<KIND_PLAYGROUND, VIS, LAYOUT>;
+    case KIND_GOTODOOR: return (StepKernel)k_step<KIND_GOTODOOR, VIS, LAYOUT>;
+    case KIND_FETCH: return (StepKernel)k_step<KIND_FETCH, VIS, LAYOUT>;
+    case KIND_REDBLUEDOORS: return (StepKernel)k_step<KIND_REDBLUEDOORS, VIS, LAYOUT>;
+    case KIND_GOTOOBJECT: return (StepKernel)k_step<KIND_GOTOOBJECT, VIS, LAYOUT>;
+    case KIND_PUTNEAR: return (StepKernel)k_step<KIND_PUTNEAR, VIS, LAYOUT>;
+    case KIND_MEMORY: return (StepKernel)k_step<KIND_MEMORY, VIS, LAYOUT>;
+    case KIND_DYNOBS: return (StepKernel)k_step<KIND_DYNOBS, VIS, LAYOUT>;
+    case KIND_ROOMGRID: return (StepKernel)k_step<KIND_ROOMGRID, VIS, LAYOUT>;
+    default: return (StepKernel)k_step<KIND_FOURROOMS, VIS, LAYOUT>;
   }
 }
-template <int MODE>
+template <int LAYOUT>
 static StepKernel pick_vis(int kind, int vis) {
-  if (vis == VIS_NONE) return pick_kind<VIS_NONE, MODE>(kind);
-  if (vis == VIS_ALU) return pick_kind<VIS_ALU, MODE>(kind);
-  return pick_kind<VIS_TBL, MODE>(kind);
+  return vis == VIS_NONE ? pick_kind<VIS_NONE, LAYOUT>(kind) : pick_kind<VIS_TBL, LAYOUT>(kind);
 }
 
 StepKernel step_kernel_window(int kind, int vis);  // mg_step_window.cu
-StepKernel step_kernel_tiled1(int kind, int vis);  // mg_step_tiled1.cu
 
 }  // namespace mg

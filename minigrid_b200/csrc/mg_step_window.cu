@@ -3,7 +3,7 @@
 
 namespace mg {
 
-StepKernel step_kernel_window(int kind, int vis) { return pick_vis<MODE_WINDOW>(kind, vis); }
+StepKernel step_kernel_window(int kind, int vis) { return pick_vis<LAYOUT_WINDOW>(kind, vis); }
 
 #ifdef MG_TIMELINE
 int debug_timeline_window(void *out) { return (int)cudaMemcpyFromSymbol(out, g_tl, sizeof(g_tl)); }

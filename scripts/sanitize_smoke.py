@@ -1,5 +1,5 @@
-"""A small, fixed workload for compute-sanitizer (memcheck / racecheck / synccheck): every K1 mode (tiled with one and
-two buffers, window), both autoreset modes with episodes forced to end (sparse and whole-tile waves), ragged last tile,
+"""A small, fixed workload for compute-sanitizer (memcheck / racecheck / synccheck): both K1 layouts (tiled, window),
+both autoreset modes with episodes forced to end (sparse and whole-tile waves), ragged last tile,
 the reset / state / full-obs kernels and the observation-only pass. Compared with the oracle so that a sanitizer run is
 also a parity run. Usage: compute-sanitizer --tool racecheck --kernel-regex kns=2mg python scripts/sanitize_smoke.py"""
 import os
@@ -12,11 +12,11 @@ import torch
 from minigrid_b200 import MinigridVecEnv
 from oracle.oracle import OracleVecEnv
 
-cases = [("MiniGrid-DoorKey-8x8-v0", None, None), ("MiniGrid-DoorKey-8x8-v0", None, "0,2,2"), ("MiniGrid-DoorKey-8x8-v0", "1", None),
+cases = [("MiniGrid-DoorKey-8x8-v0", None, None), ("MiniGrid-DoorKey-8x8-v0", "1", None),
          ("MiniGrid-FourRooms-v0", None, None), ("MiniGrid-LavaCrossingS9N1-v0", None, None), ("MiniGrid-Empty-8x8-v0", None, None),
          ("MiniGrid-Fetch-8x8-N3-v0", None, None), ("MiniGrid-MemoryS13Random-v0", None, None),
-         # two CTAs of three warps: every warp goes through several tiles (prefetch, buffer rotation, order list)
-         ("MiniGrid-DoorKey-8x8-v0", None, "3,0,0", "2"), ("MiniGrid-FourRooms-v0", None, "3,0,0", "2"), ("MiniGrid-LavaCrossingS9N1-v0", None, "3,0,1", "2")]
+         # two CTAs of three warps: every warp goes through several tiles (mbarrier phase, prefetch, order list)
+         ("MiniGrid-DoorKey-8x8-v0", None, "3", "2"), ("MiniGrid-FourRooms-v0", None, "3", "2"), ("MiniGrid-LavaCrossingS9N1-v0", None, "3", "2")]
 if len(sys.argv) > 1:
     cases = cases[: int(sys.argv[1])]
 n, steps = 1024 + 5, 14

@@ -23,7 +23,7 @@ for n in sizes:
     for _ in range(5): g.replay()
     torch.cuda.synchronize()
     buf = np.zeros((2, 160, 16), np.uint64)
-    rc = raw.mg_debug_timeline(ctypes.c_void_p(buf.ctypes.data), 1)
+    rc = raw.mg_debug_timeline(ctypes.c_void_p(buf.ctypes.data), 0)  # DoorKey-8x8: tiled layout
     assert rc == 0, rc
     ncta = int((buf[0, :, 0] != 0).sum())
     tl = buf[:, :ncta, :].astype(np.int64)

@@ -28,8 +28,8 @@ for desync in (False, True):
     for _ in range(5): g.replay()
     torch.cuda.synchronize()
     buf = np.zeros((2, 160, 16), np.uint64)
-    mode = int(os.environ.get("TL_MODE", "1"))  # 0 tiled (1 buffer), 1 tiled (2 buffers), 2 window
-    assert raw.mg_debug_timeline(ctypes.c_void_p(buf.ctypes.data), mode) == 0
+    layout = int(os.environ.get("TL_LAYOUT", "0"))  # the env's layout: 0 tiled, 1 window
+    assert raw.mg_debug_timeline(ctypes.c_void_p(buf.ctypes.data), layout) == 0
     ncta = int((buf[0, :, 0] != 0).sum())
     tl = buf[:, :ncta, :].astype(np.int64)
     a, b = (0, 1) if tl[0, :, 0].min() < tl[1, :, 0].min() else (1, 0)
